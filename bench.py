@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            our arm (one rank per GPU under torchrun for N>1)
   python bench.py --impl reference --gpus N --steps K ...  the reference's CPU implementation of the same step
+  python bench.py ... --dump-outputs DIR                   also writes what the last timed step computed (Workload.dump)
 
 Workload (config.workload = "config2"): BASELINE.json configs[1] -- ImagePolicyModelSS('resnet34'), synthetic
 batch 256/GPU, one full training step = student forward (train-mode BN) + phase-0 L1 waypoint loss against fixed
@@ -20,8 +21,10 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "oracle"))
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree it runs from (which may be read-only)
 
 GFLOP_PER_TRAIN_IMG = 28.034      # SURVEY.md 8(d): 3 x 9.441116 - 0.289014 (no dgrad for the stem)
+DUMP_SAMPLE = 1 << 20             # parameters (and their gradients) written by --dump-outputs: 4 MB each in float32
 METRIC = "images/sec (ResNet34 160x384 waypoint train step)"
 # BASELINE.json configs -> workloads (SURVEY.md 8(d)); ALGORITHMIC conv GFLOP per training image
 WORKLOADS = {
@@ -192,9 +195,9 @@ def mem_available_gb():
 
 def run_reference(args):
     """The reference's own CPU implementation of the step (its only one: SURVEY.md 0 -- the repo ships no CUDA code) on the
-    host cores: the oracle port of the workload.  Two samples: the reference's config-1 batch (8) over `steps` iterations,
-    and -- memory permitting -- the like-for-like batch of our arm (256) over a few iterations; `value` is the like-for-like
-    one when it ran."""
+    host cores: the oracle port of the workload.  Two samples, each `steps` timed iterations after `warmup` untimed ones: the
+    reference's config-1 batch (8), and -- memory permitting -- the like-for-like batch of our arm (256, ~10 s per iteration
+    on 32 threads); `value` is the like-for-like one when it ran."""
     import torch
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
@@ -202,13 +205,13 @@ def run_reference(args):
     wl = WORKLOADS[args.workload]
     cores = cpu_threads()
     torch.set_num_threads(cores)
-    rate8, sec8 = cpu_step_rate(torch, args.workload, 8, max(1, min(args.warmup, 2)), max(1, min(args.steps, 20)), cores)
+    rate8, sec8 = cpu_step_rate(torch, args.workload, 8, args.warmup, args.steps, cores)
     rate, sec, B = rate8, sec8, 8
     like = None
     if args.batch > 8 and mem_available_gb() > 120 and os.environ.get("LBC_CPU_LIKE_FOR_LIKE", "1") != "0":
-        try:    # ~35 GB of autograd state at batch 256; a handful of iterations (each ~10 s on 32 threads)
-            r, s_ = cpu_step_rate(torch, args.workload, args.batch, 1, 3, cores)
-            like = dict(value=r, batch_per_step=args.batch, sec_per_step=s_, timed_steps=3)
+        try:    # ~35 GB of autograd state at batch 256
+            r, s_ = cpu_step_rate(torch, args.workload, args.batch, args.warmup, args.steps, cores)
+            like = dict(value=r, batch_per_step=args.batch, sec_per_step=s_, timed_steps=args.steps)
             rate, sec, B = r, s_, args.batch
         except Exception as e:     # never let the optional sample take the arm down
             like = dict(error=str(e)[:200])
@@ -220,7 +223,7 @@ def run_reference(args):
                config=dict(workload=args.workload, model=wl["model"], step=wl["step"], batch_per_step=B, batch_per_gpu=B,
                            global_batch=B),
                cpu_baseline=dict(value=rate, unit="images/s", cores=torch.get_num_threads(), kind="port", sample=sample,
-                                 batch8=dict(value=rate8, sec_per_step=sec8), like_for_like=like),
+                                 batch8=dict(value=rate8, sec_per_step=sec8, timed_steps=args.steps), like_for_like=like),
                e2e=dict(value=rate, unit="images/s", h2d_bytes_per_step=0, d2h_bytes_per_step=0))
     print(json.dumps(out))
 
@@ -267,16 +270,19 @@ class Workload:
     def step_from(self, rgb, bev, speed, oh, target, loc):
         torch = self.torch
         if self.name == "config5":
-            pred = self.net(bev, speed, oh)[0]
+            pred, preds = self.net(bev, speed, oh)
             loss = self.crit(pred, loc).mean()
+            self.outputs = dict(pred=pred, preds=preds, loss=loss)
         elif self.name == "config3":
             with torch.no_grad():
                 _, t_preds = self.teacher(bev, speed, oh)
-            _, preds = self.net(rgb, speed, oh)
+            pred, preds = self.net(rgb, speed, oh)
             loss = self.crit(self.conv(preds), t_preds).mean()
+            self.outputs = dict(pred=pred, preds=preds, teacher_preds=t_preds, loss=loss)
         else:
-            pred, _ = self.net(rgb, speed, oh)
+            pred, preds = self.net(rgb, speed, oh)
             loss = self.crit(pred, target).mean()
+            self.outputs = dict(pred=pred, preds=preds, loss=loss)
         self.opt.zero_grad()
         self.dp.backward(loss)
         self.dp.step_after_backward()
@@ -294,6 +300,26 @@ class Workload:
 
     def h2d_bytes(self, u8):
         return sum(t.numel() * t.element_size() for t in self.host_batch(u8) if t is not None)
+
+    def dump(self, directory):
+        """--dump-outputs: what the last step handed its caller, as DIR/<name>.npy in float32 -- the predictions and loss
+        (outputs of step_from), the floating-point buffers (BatchNorm running statistics), and the parameters and gradients
+        the step left behind, sampled at DUMP_SAMPLE positions of the flattened parameters() (seed 0: the same positions on
+        every run; a parameter the loss does not reach has gradient zero).  About 8 MB, whatever the batch."""
+        import numpy as np
+        torch = self.torch
+        params = list(self.net.parameters())
+        flat_p = torch.cat([p.detach().reshape(-1) for p in params]).float()
+        grads = [p.grad if p.grad is not None else torch.zeros_like(p) for p in params]
+        flat_g = torch.cat([g.detach().reshape(-1) for g in grads]).float()
+        idx = torch.randperm(flat_p.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE].sort().values
+        idx = idx.to(flat_p.device)
+        arrays = {k: v.detach().float() for k, v in self.outputs.items()}
+        bufs = [b.detach().reshape(-1).float() for b in self.net.buffers() if b.dtype.is_floating_point]
+        arrays.update(params_sample=flat_p[idx], grads_sample=flat_g[idx], buffers=torch.cat(bufs))
+        os.makedirs(directory, exist_ok=True)
+        for name, a in arrays.items():
+            np.save(os.path.join(directory, name + ".npy"), a.cpu().numpy())
 
 
 def run_ours(args):
@@ -372,6 +398,8 @@ def run_ours(args):
     barrier()
     if rank == 0:
         sampler.end()
+        if args.dump_outputs:       # before any later step overwrites the state the last timed step left
+            w.dump(args.dump_outputs)
     ms = e0.elapsed_time(e1)
     launches = L.lbc_kernel_launch_count() - n0
     t = torch.tensor([ms], device=dev)
@@ -384,7 +412,7 @@ def run_ours(args):
     # inside the timed region (on the package's CudaPrefetcher side stream, overlapping the previous step's compute)
     # and the step's loss is read back device->host.
     from learningbycheating_b200.data import CudaPrefetcher
-    e2e_steps = max(5, min(args.steps, 40))    # same K as the device-resident loop (pipeline fill/drain is inside the region)
+    e2e_steps = args.steps      # same K as the device-resident loop (pipeline fill/drain is inside the region)
 
     def host_batches(n, u8):
         for _ in range(n):
@@ -525,7 +553,13 @@ def main():
                     "single all-reduce after backward (measured equal-to-slightly-slower on 2 GPUs: distributed.py)")
     ap.add_argument("--pair", type=int, default=-1, help="kernel variants: bit 0 = CTA-pair (cta_group::2) implicit-GEMM kernels, "
                                                          "bit 1 = row-of-taps weight gradient (default: LBC_PAIR)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed to "
+                    "DIR/<name>.npy (float32; inputs are seeded, so two builds can be compared output for output)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of our arm's step; the reference arm has none to write")
     if args.impl == "reference":
         run_reference(args)
     else:

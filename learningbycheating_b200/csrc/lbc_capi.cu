@@ -527,13 +527,13 @@ int lbc_op_conv_wgrad(const float* x, const float* dy, float* dw_ref, int N, int
       ref::conv_wgrad<float>(s, x, dy, dw_ref, N, H, W, Ci, Co, K, stride, pad, c.OH, c.OW, ws, wsn);
     } else if (precision == PREC_F32TC) {
       fast::TcWork tw = make_tcwork(t, nx * 4, ny * 4);
-      LBC_CHECK(fast::conv_wgrad_tc(c, x, nullptr, dy, dw_ref, N, fast::TC_BF16, fast::TC_BF16, ws, wsn, tw, s),
+      LBC_CHECK(fast::conv_wgrad_tc(c, x, nullptr, dy, dw_ref, N, fast::TC_BF16, fast::TC_BF16, tw, s),
                 "conv_wgrad_tc declined the shape");
     } else {
       bf16 *xb = t.get<bf16>(nx), *yb = t.get<bf16>(ny);
       ref::cast<float, bf16>(s, x, xb, nx);
       ref::cast<float, bf16>(s, dy, yb, ny);
-      if (!fast::conv_wgrad<bf16>(c, xb, yb, dw_ref, N, ws, wsn, s))
+      if (!fast::conv_wgrad<bf16>(c, xb, yb, dw_ref, N, s))
         ref::conv_wgrad<bf16>(s, xb, yb, dw_ref, N, H, W, Ci, Co, K, stride, pad, c.OH, c.OW, ws, wsn);
     }
     sync_stream(s);
@@ -977,7 +977,7 @@ int lbc_op_stem(const float* img, const uint8_t* img_u8, int layout, const float
         int64_t wsn = 4 << 20;
         float *ws = t.get<float>(wsn), *dwc = t.get<float>((int64_t)64 * Kp);
         LBC_CHECK(fast::tc_stem_im2col(x0, tw.a16, N, C, H, W, OH, OW, Kp, fast::TC_BF16, s), "tc_stem_im2col unavailable");
-        LBC_CHECK(fast::conv_wgrad_tc(g, nullptr, tw.a16, dy, dwc, N, fast::TC_BF16, fast::TC_BF16, ws, wsn, tw, s),
+        LBC_CHECK(fast::conv_wgrad_tc(g, nullptr, tw.a16, dy, dwc, N, fast::TC_BF16, fast::TC_BF16, tw, s),
                   "stem weight gradient (tc) declined the shape");
         LBC_CHECK(fast::stem_unpack_wgrad(dwc, dw, C, Kp, s), "stem_unpack_wgrad failed");
       }
@@ -1018,7 +1018,7 @@ int lbc_op_stem(const float* img, const uint8_t* img_u8, int layout, const float
         int64_t wsn = 4 << 20;
         float *ws = t.get<float>(wsn), *dwc = t.get<float>((int64_t)64 * Kp);
         ref::cast<float, bf16>(s, dy, dyb, ny);
-        LBC_CHECK(fast::conv_wgrad<bf16>(g, col, dyb, dwc, N, ws, wsn, s), "stem weight-gradient GEMM declined the shape");
+        LBC_CHECK(fast::conv_wgrad<bf16>(g, col, dyb, dwc, N, s), "stem weight-gradient GEMM declined the shape");
         LBC_CHECK(fast::stem_unpack_wgrad(dwc, dw, C, Kp, s), "stem_unpack_wgrad failed");
       }
     }

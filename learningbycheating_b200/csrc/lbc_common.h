@@ -208,6 +208,19 @@ extern int g_wgrad_overlap;   // schedule of backward() in the bf16 mode (lbc_ne
 extern int g_pdl;
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
+// dst[i] = src[i] + src[n + i] + ... + src[(slices - 1) * n + i], added in that order: the reduction of per-split (or
+// per-block) partials that keeps a split computation bitwise reproducible from run to run, where atomics into one
+// buffer would add the partials in whatever order the blocks finish
+template <typename T>
+__global__ void sum_slices_kernel(const T* __restrict__ src, T* __restrict__ dst, int64_t n, int slices) {
+  pdl_wait();
+  pdl_trigger();
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  T a = src[i];
+  for (int s = 1; s < slices; ++s) a += src[(int64_t)s * n + i];
+  dst[i] = a;
+}
 struct LaunchCfg {
   cudaLaunchConfig_t cfg;
   cudaLaunchAttribute attr[2];

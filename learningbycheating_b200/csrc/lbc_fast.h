@@ -68,17 +68,15 @@ inline bool conv_dgrad_ds<bf16>(const ConvL& c1, const bf16* dy1, const bf16* dy
   if (!enabled()) return false;
   return conv_dgrad_ds_bf16(c1, dy1, dy_ds, dx, B, s);
 }
-bool conv_wgrad_bf16(const ConvL& c, const bf16* x, const bf16* dy, float* dw_ref, int B, float* scratch,
-                     int64_t scratch_floats, lbc_stream_t s);
+bool conv_wgrad_bf16(const ConvL& c, const bf16* x, const bf16* dy, float* dw_ref, int B, lbc_stream_t s);
 template <class T>
-inline bool conv_wgrad(const ConvL&, const T*, const T*, float*, int, float*, int64_t, lbc_stream_t) {
+inline bool conv_wgrad(const ConvL&, const T*, const T*, float*, int, lbc_stream_t) {
   return false;
 }
 template <>
-inline bool conv_wgrad<bf16>(const ConvL& c, const bf16* x, const bf16* dy, float* dw_ref, int B, float* scratch,
-                             int64_t scratch_floats, lbc_stream_t s) {
+inline bool conv_wgrad<bf16>(const ConvL& c, const bf16* x, const bf16* dy, float* dw_ref, int B, lbc_stream_t s) {
   if (!enabled()) return false;
-  return conv_wgrad_bf16(c, x, dy, dw_ref, B, scratch, scratch_floats, s);
+  return conv_wgrad_bf16(c, x, dy, dw_ref, B, s);
 }
 
 // ---- fp32tc: parity-grade tensor-core convolutions over fp32 NHWC tensors (lbc_fast_conv.cu) --------------------
@@ -105,7 +103,7 @@ bool conv_dgrad_tc(const ConvL& c, const float* dy, const float* dy_ds, float* d
                    int dy_fmt, const TcWork& w, lbc_stream_t s);
 // dw_ref [Co][Ci][K][K] = sum_pixels dy x;  x16 != null: x already split (stem column tensor, in w.a16)
 bool conv_wgrad_tc(const ConvL& c, const float* x, const void* x16, const float* dy, float* dw_ref, int B, int x_fmt, int dy_fmt,
-                   float* scratch, int64_t scratch_floats, const TcWork& w, lbc_stream_t s);
+                   const TcWork& w, lbc_stream_t s);
 // stem: x0 [B,H,W,C] fp32 NHWC -> split column tensor [B*OH*OW][hi Kp | lo Kp] (k = (kh*7+kw)*C + c, zero padded)
 bool tc_stem_im2col(const float* x0, void* col16, int B, int C, int H, int W, int OH, int OW, int Kp, int fmt, lbc_stream_t s);
 

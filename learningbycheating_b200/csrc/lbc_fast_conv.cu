@@ -1403,7 +1403,7 @@ struct StemWgradParams {
   int TW, TH, TN, tiles_w, tiles_h, tiles_n;
   int k_tiles, k_per_split, splits;
   int C;           // real input channels (<= 4)
-  float* dw_ref;   // [64][C][7][7] fp32, pre-zeroed
+  float* dw_ref;   // [splits][64][C][7][7] fp32 partials: every element stored once per split (summed in split order)
 };
 __device__ __forceinline__ uint64_t umma_desc_mn_sw64(uint32_t smem_addr, uint32_t lbo_bytes) {
   uint64_t d = 0;
@@ -1531,7 +1531,7 @@ stem_wgrad_kernel(const __grid_constant__ CUtensorMap mDY, const __grid_constant
 #pragma unroll
         for (int j = 0; j < 32; ++j) {
           const int co = ch * 32 + j;
-          atomicAdd(p.dw_ref + (((int64_t)co * p.C + c) * 7 + kh) * 7 + (kwp - 1), __uint_as_float(r[j]));
+          p.dw_ref[(int64_t)split * 64 * p.C * 49 + (((int64_t)co * p.C + c) * 7 + kh) * 7 + (kwp - 1)] = __uint_as_float(r[j]);
         }
       }
     }
@@ -1944,7 +1944,9 @@ static void launch_stem_wgrad(const CUtensorMap& mDY, const CUtensorMap& mX0, co
   LBC_LAUNCHED(CH == 4 ? "stem_wgrad_kernel" : CH == 8 ? "stem_wgrad_kernel<8ch>" : "stem_wgrad_kernel<s2d>");
   LBC_CUDA(cudaGetLastError());
 }
-// dw_ref[64][C][7][7] = sum_pixels dy x window(x4); dw_ref is zeroed here
+template <int Slot>
+static float* wgrad_partials(int64_t floats);
+// dw_ref[64][C][7][7] = sum_pixels dy x window(x4), the K splits' partial sums added in split order
 bool stem_wgrad_bf16(const bf16* x4, const bf16* dy, float* dw_ref, int B, int C, int H, int W, int OH, int OW, lbc_stream_t s,
                      int CH) {
   if ((H % 2) || (W % 2) || OH * 2 != H || OW * 2 != W || C > stem_x_ch(CH) || (CH != 4 && CH != 8 && CH != 16)) return false;
@@ -1960,20 +1962,24 @@ bool stem_wgrad_bf16(const bf16* x4, const bf16* dy, float* dw_ref, int B, int C
   p.k_per_split = (p.k_tiles + splits - 1) / splits;
   p.splits = (p.k_tiles + p.k_per_split - 1) / p.k_per_split;
   p.C = C;
-  p.dw_ref = dw_ref;
+  const int64_t slice = (int64_t)64 * C * 49;
+  p.dw_ref = wgrad_partials<2>((int64_t)p.splits * slice);
+  if (!p.dw_ref) return false;
   const int64_t pitch = CH == 16 ? (int64_t)(W + 8) * 16 : (int64_t)(W + 8) * CH * 2;
   const int64_t img = (int64_t)(W + 8) * (H + 6) * stem_x_ch(CH) * 2;
   CUtensorMap mX0 = make_map_stem(x4, OW, (H + 6) / 2, B, pitch, img, p.TW, p.TH, p.TN, CH);
   CUtensorMap mX1 = make_map_stem((const uint8_t*)x4 + pitch, OW, (H + 6) / 2, B, pitch, img, p.TW, p.TH, p.TN, CH);
   const int64_t eb = 2;
   CUtensorMap mDY = make_map_4d(dy, 64, OW, OH, B, 64 * eb, (int64_t)OW * 64 * eb, (int64_t)OH * OW * 64 * eb, p.TW, p.TH, p.TN);
-  LBC_CUDA(cudaMemsetAsync(dw_ref, 0, sizeof(float) * 64 * C * 49, s));
   if (CH == 4)
     launch_stem_wgrad<4>(mDY, mX0, mX1, p, s);
   else if (CH == 8)
     launch_stem_wgrad<8>(mDY, mX0, mX1, p, s);
   else
     launch_stem_wgrad<16>(mDY, mX0, mX1, p, s);
+  { auto k_ = sum_slices_kernel<float>; LBC_LAUNCH(k_, dim3((unsigned)((slice + 255) / 256)), dim3(256), 0, s, (const float*)p.dw_ref, dw_ref, slice, p.splits); }
+  LBC_LAUNCHED("sum_slices_kernel");
+  LBC_CUDA(cudaGetLastError());
   return true;
 }
 
@@ -2171,8 +2177,8 @@ static bool conv_dgrad_impl(const ConvL& c, const void* dy_v, const void* wt, co
 //   D[128 co x BNW ci] (fp32, TMEM) += A[128 co x 128 pixels] * B[BNW ci x 128 pixels]^T, both operands "MN-major":
 //   a TMA box {64 ch, TW, TH, TN} lands as [128 pixels][64 ch] rows of 128 B (128 B swizzle) = the UMMA MN-major
 //   SWIZZLE_128B canonical layout with K = pixels (8-row groups 1024 B apart, 64-channel blocks LBO apart).
-//   One CTA per (co tile, tap, ci tile, K split); split-K partials are reduced with fp32 red.global.add into a
-//   packed [Co][tap][Ci] scratch that a tiny kernel then permutes into the reference's [Co][Ci][kh][kw] .grad.
+//   One CTA per (co tile, tap, ci tile, K split); each split stores its partials into its own packed [Co][tap][Ci] slice,
+//   and a tiny kernel adds the slices in split order while permuting into the reference's [Co][Ci][kh][kw] .grad.
 // =============================================================================================================
 struct WgradParams {
   int TW, TH, TN, tiles_w, tiles_h, tiles_n;
@@ -2180,7 +2186,7 @@ struct WgradParams {
   int co_tiles, ci_tiles, num_taps;
   int tap_dh[9], tap_dw[9], tap_map[9];
   int Co, Ci;
-  float* out;  // [Co][num_taps][Ci] fp32, pre-zeroed
+  float* out;  // [splits][Co][num_taps][Ci] fp32 partials, every element stored once per split
   // swap mode (Co == 64): M = two (tap, 64-channel ci chunk) combos of x, N = the 64 output channels of dy, so the
   // 128-row MMA is full instead of half zero padding
   int swap, num_combos, chunks_per_tap;
@@ -2346,6 +2352,7 @@ wgrad_gemm_kernel(const __grid_constant__ CUtensorMap mDY, const __grid_constant
     mbar_wait(tfull, 0);
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16);
+    float* out = p.out + (int64_t)split * p.Co * p.num_taps * p.Ci;
 #pragma unroll 1
     for (int ch = 0; ch < BNW / 32; ++ch) {
       uint32_t r[32];
@@ -2360,13 +2367,13 @@ wgrad_gemm_kernel(const __grid_constant__ CUtensorMap mDY, const __grid_constant
 #pragma unroll
           for (int j = 0; j < 32; ++j) {
             const int con = ch * 32 + j;   // output channel
-            atomicAdd(p.out + ((int64_t)con * p.num_taps + tp) * p.Ci + ci, __uint_as_float(r[j]));
+            out[((int64_t)con * p.num_taps + tp) * p.Ci + ci] = __uint_as_float(r[j]);
           }
         }
       } else if (co < p.Co) {
-        float* dst = p.out + ((int64_t)co * p.num_taps + tap) * p.Ci + ci_tile * BNW + ch * 32;
+        float* dst = out + ((int64_t)co * p.num_taps + tap) * p.Ci + ci_tile * BNW + ch * 32;
 #pragma unroll
-        for (int j = 0; j < 32; ++j) atomicAdd(dst + j, __uint_as_float(r[j]));
+        for (int j = 0; j < 32; ++j) dst[j] = __uint_as_float(r[j]);
       }
     }
   }
@@ -2833,8 +2840,9 @@ __global__ void __launch_bounds__(144 * kRedGroups) wgrad3_reduce_kernel(const f
   }
 }
 
-// packed fp32 [Co][taps][Ci] -> reference layout [Co][Ci][K][K]
-__global__ void wgrad_unpack_kernel(const float* __restrict__ src, float* __restrict__ dst, int Co, int Ci, int KK) {
+// packed fp32 [splits][Co][taps][Ci] -> reference layout [Co][Ci][K][K], the splits added in order
+__global__ void wgrad_unpack_kernel(const float* __restrict__ src, float* __restrict__ dst, int Co, int Ci, int KK,
+                                    int splits) {
   pdl_wait();
   pdl_trigger();
   int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -2844,7 +2852,10 @@ __global__ void wgrad_unpack_kernel(const float* __restrict__ src, float* __rest
   int64_t r = i / KK;
   int ci = (int)(r % Ci);
   int co = (int)(r / Ci);
-  dst[i] = src[((int64_t)co * KK + t) * Ci + ci];
+  const float* sp = src + ((int64_t)co * KK + t) * Ci + ci;
+  float a = sp[0];
+  for (int k = 1; k < splits; ++k) a += sp[(int64_t)k * n];
+  dst[i] = a;
 }
 
 template <int BNW, int STAGES>
@@ -2863,7 +2874,10 @@ static void launch_wgrad(const CUtensorMap& mDY, const CUtensorMap* mX, const Wg
 
 // bit 1 of the pair/variant mode (LBC_PAIR / lbc_set_fast_kernels bit 4): row-of-taps weight-gradient kernel
 // (bit 2: its CTA-pair variant where Co % 256 == 0)
-static float* wgrad3_partials(int64_t floats) {   // [splits][Co][9][Ci] scratch, grown on demand (single stream)
+// split-K partial scratch, grown on demand; one buffer per kind of split computation, each used from one stream at a time
+// (Slot 0: row-of-taps weight gradient [splits][Co][9][Ci], 1: wgrad_gemm [splits][Co][taps][Ci], 2: stem [splits][64][C][49])
+template <int Slot>
+static float* wgrad_partials(int64_t floats) {
   static float* buf = nullptr;
   static int64_t cap = 0;
   if (floats > cap) {
@@ -2944,7 +2958,7 @@ static bool try_wgrad9(const ConvL& c, const bf16* x, const bf16* dy, float* dw_
   p.k_per_split = (p.k_tiles + splits - 1) / splits;
   splits = (p.k_tiles + p.k_per_split - 1) / p.k_per_split;
   const int64_t wsize = (int64_t)64 * 9 * 64;
-  p.out = wgrad3_partials((int64_t)splits * wsize);
+  p.out = wgrad_partials<0>((int64_t)splits * wsize);
   if (!p.out) return false;
   const int64_t eb = 2;
   CUtensorMap mDY = make_map_4d(dy, 64, c.W, c.H, B, 64 * eb, (int64_t)c.W * 64 * eb, (int64_t)c.H * c.W * 64 * eb, 8, p.TH, p.TN);
@@ -2963,9 +2977,8 @@ static bool try_wgrad9(const ConvL& c, const bf16* x, const bf16* dy, float* dw_
   LBC_LAUNCHED("wgrad3_reduce_kernel");
   return true;
 }
-static bool try_wgrad3(const ConvL& c, const bf16* x, const bf16* dy, float* dw_ref, int B, float* scratch, lbc_stream_t s,
+static bool try_wgrad3(const ConvL& c, const bf16* x, const bf16* dy, float* dw_ref, int B, lbc_stream_t s,
                        const GemmMode& m) {
-  (void)scratch;
   if (!(g_pair_mode & 2)) return false;
   const int CX = m.split ? 2 * c.Ci : c.Ci, CY = m.split ? 2 * c.Co : c.Co;   // channels of the stored x / dy tensors
   const bool pair = (g_pair_mode & 4) && (c.Co % 256 == 0);
@@ -3035,7 +3048,7 @@ static bool try_wgrad3(const ConvL& c, const bf16* x, const bf16* dy, float* dw_
     }
   }
   const int64_t wsize = (int64_t)c.Co * 9 * c.Ci;
-  p.out = wgrad3_partials((int64_t)p.splits * wsize);
+  p.out = wgrad_partials<0>((int64_t)p.splits * wsize);
   if (!p.out) return false;
   const int grid = p.splits * out_tiles;   // pair: consecutive blocks (2c, 2c+1) form the cluster of co tiles (2c', 2c'+1)
   if (pair)
@@ -3048,17 +3061,16 @@ static bool try_wgrad3(const ConvL& c, const bf16* x, const bf16* dy, float* dw_
   return true;
 }
 
-// x [B,H,W,Ci], dy [B,OH,OW,Co] -> dw_ref fp32 [Co][Ci][K][K]; scratch >= Co*K*K*Ci floats
+// x [B,H,W,Ci], dy [B,OH,OW,Co] -> dw_ref fp32 [Co][Ci][K][K]
 // (split mode: x [B,H,W,2Ci], dy [B,OH,OW,2Co] as hi | lo planes; fmt_a = format of dy, fmt_b = format of x)
-static bool conv_wgrad_impl(const ConvL& c, const bf16* x, const bf16* dy, float* dw_ref, int B, float* scratch,
-                            int64_t scratch_floats, lbc_stream_t s, const GemmMode& m) {
+static bool conv_wgrad_impl(const ConvL& c, const bf16* x, const bf16* dy, float* dw_ref, int B, lbc_stream_t s,
+                            const GemmMode& m) {
   if (!supported(c)) return false;
   if (m.split && c.Co != 64 && (c.Co % 128)) return false;   // the 128-row dy tile must not run into the lo plane
   const int KK = c.K * c.K;
   const int64_t wsize = (int64_t)c.Co * KK * c.Ci;
-  if (wsize > scratch_floats) return false;
   if (try_wgrad9(c, x, dy, dw_ref, B, s, m)) return true;
-  if (try_wgrad3(c, x, dy, dw_ref, B, scratch, s, m)) return true;
+  if (try_wgrad3(c, x, dy, dw_ref, B, s, m)) return true;
   const int CX = m.split ? 2 * c.Ci : c.Ci, CY = m.split ? 2 * c.Co : c.Co;
   WgradParams p;
   memset(&p, 0, sizeof(p));
@@ -3084,7 +3096,6 @@ static bool conv_wgrad_impl(const ConvL& c, const bf16* x, const bf16* dy, float
   p.num_taps = KK;
   p.Co = c.Co;
   p.Ci = c.Ci;
-  p.out = scratch;
   p.chunks_per_tap = c.Ci / 64;
   p.num_combos = KK * p.chunks_per_tap;
   const int out_tiles = p.swap ? (p.num_combos + 1) / 2 : p.co_tiles * p.ci_tiles * KK;
@@ -3135,20 +3146,20 @@ static bool conv_wgrad_impl(const ConvL& c, const bf16* x, const bf16* dy, float
         p.tap_map[t] = a * 2 + b;
       }
   }
-  LBC_CUDA(cudaMemsetAsync(scratch, 0, sizeof(float) * wsize, s));
+  p.out = wgrad_partials<1>((int64_t)p.splits * wsize);
+  if (!p.out) return false;
   if (BNW == 128)
     launch_wgrad<128, 3>(mDY, mX, p, s);
   else
     launch_wgrad<64, 4>(mDY, mX, p, s);
   int64_t n = wsize;
-  { auto k_ = wgrad_unpack_kernel; LBC_LAUNCH(k_, dim3((unsigned)((n + 255) / 256)), dim3(256), 0, s, scratch, dw_ref, c.Co, c.Ci, KK); }
+  { auto k_ = wgrad_unpack_kernel; LBC_LAUNCH(k_, dim3((unsigned)((n + 255) / 256)), dim3(256), 0, s, (const float*)p.out, dw_ref, c.Co, c.Ci, KK, p.splits); }
   LBC_LAUNCHED("wgrad_unpack_kernel");
   LBC_CUDA(cudaGetLastError());
   return true;
 }
-bool conv_wgrad_bf16(const ConvL& c, const bf16* x, const bf16* dy, float* dw_ref, int B, float* scratch,
-                     int64_t scratch_floats, lbc_stream_t s) {
-  return conv_wgrad_impl(c, x, dy, dw_ref, B, scratch, scratch_floats, s, GemmMode());
+bool conv_wgrad_bf16(const ConvL& c, const bf16* x, const bf16* dy, float* dw_ref, int B, lbc_stream_t s) {
+  return conv_wgrad_impl(c, x, dy, dw_ref, B, s, GemmMode());
 }
 
 // =============================================================================================================
@@ -3284,7 +3295,7 @@ bool conv_dgrad_tc(const ConvL& c, const float* dy, const float* dy_ds, float* d
                          tc_mode(dy_fmt, dy_fmt, 1.0f / kTcWeightScale));   // c.wpt16 / c.wcomb16 split in dy_fmt
 }
 bool conv_wgrad_tc(const ConvL& c, const float* x, const void* x16, const float* dy, float* dw_ref, int B, int x_fmt, int dy_fmt,
-                   float* scratch, int64_t scratch_floats, const TcWork& w, lbc_stream_t s) {
+                   const TcWork& w, lbc_stream_t s) {
   if (!enabled() || !supported(c) || x_fmt != dy_fmt) return false;   // one operand format per MMA
   const int64_t rx = (int64_t)B * c.H * c.W, ry = (int64_t)B * c.OH * c.OW;
   if (ry * c.Co * 4 > w.b_bytes) return false;
@@ -3294,13 +3305,13 @@ bool conv_wgrad_tc(const ConvL& c, const float* x, const void* x16, const float*
     x16 = w.a16;
   }
   if (!tc_split(dy, w.b16, ry, c.Co, dy_fmt, 1.0f, s)) return false;
-  return conv_wgrad_impl(c, (const bf16*)x16, (const bf16*)w.b16, dw_ref, B, scratch, scratch_floats, s, tc_mode(dy_fmt, x_fmt, 1.0f));
+  return conv_wgrad_impl(c, (const bf16*)x16, (const bf16*)w.b16, dw_ref, B, s, tc_mode(dy_fmt, x_fmt, 1.0f));
 }
 
 #else   // LBC_HOST_EMU: no tensor cores on the host; the executor runs the correctness-first kernels
 bool conv_fwd_bf16(const ConvL&, const bf16*, bf16*, int, const float*, lbc_stream_t, float*, int*) { return false; }
 bool conv_dgrad_bf16(const ConvL&, const bf16*, bf16*, int, const float*, bool, lbc_stream_t) { return false; }
-bool conv_wgrad_bf16(const ConvL&, const bf16*, const bf16*, float*, int, float*, int64_t, lbc_stream_t) { return false; }
+bool conv_wgrad_bf16(const ConvL&, const bf16*, const bf16*, float*, int, lbc_stream_t) { return false; }
 bool conv_dgrad_ds_bf16(const ConvL&, const bf16*, const bf16*, bf16*, int, lbc_stream_t) { return false; }
 void set_c64_variant(bool) {}
 void set_pair_mode(int) {}
@@ -3311,7 +3322,7 @@ bool stem_wgrad_bf16(const bf16*, const bf16*, float*, int, int, int, int, int, 
 bool tc_split(const float*, void*, int64_t, int, int, float, lbc_stream_t) { return false; }
 bool conv_fwd_tc(const ConvL&, const float*, const void*, float*, int, const float*, bool, int, const TcWork&, lbc_stream_t) { return false; }
 bool conv_dgrad_tc(const ConvL&, const float*, const float*, float*, int, const float*, bool, int, const TcWork&, lbc_stream_t) { return false; }
-bool conv_wgrad_tc(const ConvL&, const float*, const void*, const float*, float*, int, int, int, float*, int64_t, const TcWork&, lbc_stream_t) { return false; }
+bool conv_wgrad_tc(const ConvL&, const float*, const void*, const float*, float*, int, int, int, const TcWork&, lbc_stream_t) { return false; }
 bool tc_stem_im2col(const float*, void*, int, int, int, int, int, int, int, int, lbc_stream_t) { return false; }
 #endif
 

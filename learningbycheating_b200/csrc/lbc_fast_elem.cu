@@ -138,11 +138,12 @@ __global__ void __launch_bounds__(256, 6) bn_stats_kernel(const uint4* __restric
     }
   }
 }
-// sums[col] (+)= sum_p partial[p][col] for col < 2C.  32 columns x 32 partial-lanes per block (1024 threads); when there
-// are many partial rows (conv-epilogue statistics: one row per 128-pixel tile) the rows are split over blockIdx.y and
-// the (<= 32) block results are combined with one fp32 atomic each into the pre-zeroed sums.
-__global__ void __launch_bounds__(1024) col_finalize_kernel(const float* __restrict__ partial, int P, int C2, float* sums,
-                                                            int rows_per_block, int use_atomic) {
+// out[blockIdx.y][col] = sum_p partial[p][col] for col < 2C.  32 columns x 32 partial-lanes per block (1024 threads); when
+// there are many partial rows (conv-epilogue statistics: one row per 128-pixel tile) the rows are split over blockIdx.y
+// into (<= 32) rows of block sums that sum_slices_kernel then adds in a fixed order (fp32 atomics would add them in the
+// order the blocks finish, and the statistics would change in the last bits from run to run).
+__global__ void __launch_bounds__(1024) col_finalize_kernel(const float* __restrict__ partial, int P, int C2, float* out,
+                                                            int rows_per_block) {
   pdl_wait();
   pdl_trigger();
   const int col = blockIdx.x * 32 + (threadIdx.x & 31);
@@ -160,10 +161,7 @@ __global__ void __launch_bounds__(1024) col_finalize_kernel(const float* __restr
     float t = 0.f;
 #pragma unroll
     for (int i = 0; i < 32; ++i) t += red[i][threadIdx.x & 31];
-    if (use_atomic)
-      atomicAdd(sums + col, t);
-    else
-      sums[col] = t;
+    out[(int64_t)blockIdx.y * C2 + col] = t;
   }
 }
 constexpr int64_t kPartialFloats = (int64_t)4096 * 2 * 2560;
@@ -179,14 +177,36 @@ static float* partial_buffer() {
   return p;
 }
 int64_t stat_partial_capacity() { return kPartialFloats; }
+static float* block_sums_buffer() {   // [32][2C] rows of col_finalize block sums (C2 <= 2 x 2560, as the partial rows)
+  static float* p = [] {
+    void* q = nullptr;
+    if (cudaMalloc(&q, sizeof(float) * 32 * 2 * 2560) != cudaSuccess) {
+      cudaGetLastError();
+      q = nullptr;
+    }
+    return (float*)q;
+  }();
+  return p;
+}
 static void col_finalize(const float* partial, int P, int C2, float* sums, lbc_stream_t s) {
   int rb = P / 512;          // >= 512 rows per block (16 per thread) before splitting
   if (rb > 32) rb = 32;
   if (rb < 1) rb = 1;
   const int rows_per_block = (P + rb - 1) / rb;
   rb = (P + rows_per_block - 1) / rows_per_block;
-  if (rb > 1) cudaMemsetAsync(sums, 0, sizeof(float) * C2, s);
-  { auto k_ = col_finalize_kernel; LBC_LAUNCH(k_, dim3(dim3((C2 + 31) / 32, rb)), dim3(1024), 0, s, partial, P, C2, sums, rows_per_block, rb > 1 ? 1 : 0); }
+  float* out = sums;
+  if (rb > 1) {
+    out = block_sums_buffer();
+    LBC_CHECK(out != nullptr && C2 <= 2 * 2560, "col_finalize: no block-sum scratch for this shape");
+  }
+  { auto k_ = col_finalize_kernel; LBC_LAUNCH(k_, dim3(dim3((C2 + 31) / 32, rb)), dim3(1024), 0, s, partial, P, C2, out, rows_per_block); }
+  if (rb > 1) {
+    LBC_LAUNCHED("col_finalize_kernel");
+    auto k_ = sum_slices_kernel<float>;
+    LBC_LAUNCH(k_, dim3((C2 + 255) / 256), dim3(256), 0, s, (const float*)out, sums, (int64_t)C2, rb);
+    LBC_LAUNCHED("sum_slices_kernel");
+    return;
+  }
   LBC_LAUNCHED("col_finalize_kernel");
 }
 

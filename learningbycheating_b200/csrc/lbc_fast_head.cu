@@ -465,10 +465,11 @@ bool head_dlogits_f32(const float* logits, const float* rowmax, const float* row
   return true;
 }
 
-// S[kj][c] += sum_pix dl[n,kj,pix]*hhat[n,pix,c] (c<64), S[kj][64] += sum dl   (double atomics, S pre-zeroed):
+// S[block][kj][c] = sum_pix dl[n,kj,pix]*hhat[n,pix,c] (c<64), S[block][kj][64] = sum dl over the block's tiles:
 // D[20 -> 32][64 (+8: a tile of ones gives sum dl)] += dl[32][128 px] x H[128 px][64], K = pixels; warp w owns pixels
 // [32w, 32w+32) of every tile (K split over the warps), dl enters as hi + lo bf16 pairs, H as stored.  The accumulators
-// (raw moments sum dl*h) live across the block's tiles; at the end  S = rstd*(raw - mean * sum dl)  per block, then doubles.
+// (raw moments sum dl*h) live across the block's tiles; at the end  S = rstd*(raw - mean * sum dl)  per block, as doubles
+// that sum_slices_kernel adds in block order.
 __global__ void __launch_bounds__(128) head_s_mma_kernel(const float* __restrict__ dlogits, const bf16* __restrict__ h,
                                                          const float* __restrict__ mean, const float* __restrict__ rstd,
                                                          double* S, int N, int HW) {
@@ -571,28 +572,45 @@ __global__ void __launch_bounds__(128) head_s_mma_kernel(const float* __restrict
       const float s0 = (part[0][kj][64] + part[1][kj][64]) + (part[2][kj][64] + part[3][kj][64]);
       v = (raw - mean[c] * s0) * rstd[c];
     }
-    atomicAdd(&S[kj * 65 + c], (double)v);
+    S[(int64_t)blockIdx.x * 20 * 65 + kj * 65 + c] = (double)v;
   }
 }
 
-// S: [20][65] doubles (zeroed here).  Produces S, then the caller computes parameter grads (ref::head_param_grads),
+// S: [20][65] doubles (the blocks' partials added in block order).  Produces S, then the caller computes parameter grads (ref::head_param_grads),
 // then head_backward_dh_bf16 writes the masked d(h).
 bool head_backward_s_bf16(const float* dlogits, const bf16* h, const float* mean, const float* rstd, double* S, int N, int HW,
                           lbc_stream_t s) {
   if (!enabled()) return false;
   if (HW & 3) return false;   // (16-byte dlogits staging)
-  LBC_CUDA(cudaMemsetAsync(S, 0, sizeof(double) * 20 * 65, s));
   int grid = sm_count3() * 2;
   int ntiles = N * ((HW + 127) / 128);
   if (grid > ntiles) grid = ntiles;
+  static double* part = nullptr;   // [grid][20][65] block partials (main stream only)
+  static int part_blocks = 0;
+  if (grid > part_blocks) {
+    if (part) {
+      cudaDeviceSynchronize();
+      cudaFree(part);
+    }
+    part = nullptr;
+    part_blocks = 0;
+    if (cudaMalloc(&part, sizeof(double) * 20 * 65 * (size_t)grid) != cudaSuccess) {
+      cudaGetLastError();
+      part = nullptr;
+      return false;
+    }
+    part_blocks = grid;
+  }
   constexpr int SMEM = 32768 + 2 * 20 * 136 * 4;
   static bool configured = false;
   if (!configured) {
     LBC_CUDA(cudaFuncSetAttribute(head_s_mma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM));
     configured = true;
   }
-  { auto k_ = head_s_mma_kernel; LBC_LAUNCH(k_, dim3(grid), dim3(128), SMEM, s, dlogits, h, mean, rstd, S, N, HW); }
+  { auto k_ = head_s_mma_kernel; LBC_LAUNCH(k_, dim3(grid), dim3(128), SMEM, s, dlogits, h, mean, rstd, part, N, HW); }
   LBC_LAUNCHED("head_s_mma_kernel");
+  { auto k_ = sum_slices_kernel<double>; LBC_LAUNCH(k_, dim3((20 * 65 + 255) / 256), dim3(256), 0, s, (const double*)part, S, (int64_t)20 * 65, grid); }
+  LBC_LAUNCHED("sum_slices_kernel");
   LBC_CUDA(cudaGetLastError());
   return true;
 }

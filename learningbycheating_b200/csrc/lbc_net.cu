@@ -783,12 +783,12 @@ class Net : public NetBase {
     ProfScope ps("conv_wgrad", s, conv_flops(c, B), 0);
     if (tc) {
       (void)x_is_grad;   // either way one operand is a gradient: bf16 planes for both
-      LBC_CHECK(fast::conv_wgrad_tc(c, (const float*)x, nullptr, (const float*)dy, G + c.w_off, B, fast::TC_BF16, fast::TC_BF16, ws_f,
-                                    ws_f_n, tcw, s),
+      LBC_CHECK(fast::conv_wgrad_tc(c, (const float*)x, nullptr, (const float*)dy, G + c.w_off, B, fast::TC_BF16, fast::TC_BF16, tcw,
+                                    s),
                 "PREC_F32TC: tensor-core weight gradient unavailable for this layer");
       return;
     }
-    if (fast::conv_wgrad<T>(c, x, dy, G + c.w_off, B, ws_f, ws_f_n, s)) return;
+    if (fast::conv_wgrad<T>(c, x, dy, G + c.w_off, B, s)) return;
     ref::conv_wgrad<T>(s, x, dy, G + c.w_off, B, c.H, c.W, c.Ci, c.Co, c.K, c.stride, c.pad, c.OH, c.OW, ws_f, ws_f_n);
   }
   void bn_forward(BNL& bn, const T* x, int64_t M, const T* residual, bool relu, T* y, bool train, lbc_stream_t s,
@@ -1200,14 +1200,14 @@ class Net : public NetBase {
       LBC_CHECK(stem_wgrad_done, "stem direct weight gradient failed");
     } else if (stem_fast_used) {
       ProfScope ps("conv_wgrad", s, conv_flops(stem, B), 0);
-      if (fast::conv_wgrad<T>(stem_gemm, stem_col, tB, stem_dw_col, B, ws_f, ws_f_n, s))
+      if (fast::conv_wgrad<T>(stem_gemm, stem_col, tB, stem_dw_col, B, s))
         stem_wgrad_done = fast::stem_unpack_wgrad(stem_dw_col, G + stem.w_off, in_ch, stem_gemm.Ci, s);
     }
     if (!stem_wgrad_done && stem_tc_used) {
       ProfScope ps("conv_wgrad", s, conv_flops(stem, B), 0);
       bool ok = fast::tc_stem_im2col((const float*)x0, tcw.a16, B, in_ch, in_h, in_w, stem_oh, stem_ow, stem_gemm.Ci, fast::TC_BF16, s) &&
-                fast::conv_wgrad_tc(stem_gemm, nullptr, tcw.a16, (const float*)tB, stem_dw_col, B, fast::TC_BF16, fast::TC_BF16, ws_f,
-                                    ws_f_n, tcw, s) &&
+                fast::conv_wgrad_tc(stem_gemm, nullptr, tcw.a16, (const float*)tB, stem_dw_col, B, fast::TC_BF16, fast::TC_BF16, tcw,
+                                    s) &&
                 fast::stem_unpack_wgrad(stem_dw_col, G + stem.w_off, in_ch, stem_gemm.Ci, s);
       LBC_CHECK(ok, "PREC_F32TC: tensor-core stem weight gradient unavailable");
       stem_wgrad_done = true;

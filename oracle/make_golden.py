@@ -1,6 +1,7 @@
 """TEST INFRASTRUCTURE ONLY -- generate tests/golden/*.npz from the UNMODIFIED reference.
 
-Run in the build container (needs /root/reference):   python oracle/make_golden.py
+Needs the reference tree (LBC_REFERENCE_ROOT, see ref_import.py):   python oracle/make_golden.py [reference_forward]
+(with the argument, only tests/golden/reference_forward_B2.npz is rewritten).
 
 For each case it drives the reference's own classes (ImagePolicyModelSS, BirdViewPolicyModelSS,
 train_image_phase{0,1}.CoordConverter / LocationLoss, torch.optim.Adam) exactly as
@@ -22,6 +23,9 @@ import ref_import  # noqa: E402
 OUT = os.path.join(HERE, "..", "tests", "golden")
 N_STEPS = 3
 SMALL = 4096
+# torch's CPU kernels split their reductions by intra-op thread, so the last bits of a result depend on the thread count;
+# the golden runs were recorded with this many, and tests that replay them bit for bit set it too
+GOLDEN_THREADS = 8
 
 
 def sample_coords(shape, k=24, seed=7):
@@ -191,9 +195,35 @@ def run_birdview_case(ns, B, teacher0):
     return out
 
 
-def main():
+def state_sha256(t):
+    """Digest of a state_dict tensor's bytes: tests hold the package's initial state to the reference's, bit for bit."""
+    import hashlib
+    return hashlib.sha256(t.detach().contiguous().cpu().numpy().tobytes()).hexdigest()
+
+
+def reference_forward(ns):
+    """One train-mode forward of the reference's seed-0 student on synthetic_batch(2): its predictions, and a digest of
+    every state_dict tensor it was computed from."""
+    torch.manual_seed(0)
+    s = ns.ImagePolicyModelSS('resnet34', all_branch=True)
+    sd = s.state_dict()
+    keys, digests = np.array(list(sd.keys())), np.array([state_sha256(v) for v in sd.values()])   # before the forward
+    b = orc.synthetic_batch(2)                                                                     # updates BN buffers
+    s.train()
+    pred, preds = s(b["rgb"], b["speed"], ns.one_hot(b["command"]))
+    np.savez_compressed(os.path.join(OUT, "reference_forward_B2.npz"), pred=pred.detach().numpy().copy(),
+                        preds=preds.detach().numpy().copy(), state_keys=keys, state_sha256=digests)
+    print("reference forward written")
+
+
+def main(only=None):
     ns = ref_import.load()
     os.makedirs(OUT, exist_ok=True)
+    torch.set_num_threads(GOLDEN_THREADS)
+    if only == "reference_forward":
+        reference_forward(ns)
+        return
+    reference_forward(ns)
     torch.manual_seed(0)     # SURVEY 8(c): student first, then teacher (RNG order matters)
     student = ns.ImagePolicyModelSS('resnet34', all_branch=True)
     teacher = ns.BirdViewPolicyModelSS('resnet18', all_branch=True)
@@ -235,4 +265,4 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    main(sys.argv[1] if len(sys.argv) > 1 else None)
